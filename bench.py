@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU restatement on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1], "cfg2"): complex64 IQ at a nominal 100 MS/s, 65536-point
 Blackman-Harris main spectrum over every frame + one QPSK inspector (1 MBd, RRC 0.35, Costas + Gardner,
@@ -16,8 +17,10 @@ Prints ONE JSON line (see README / DESIGN.md section "Measurement").
 import argparse
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -25,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (it may be read-only)
 
 N_FFT = 65536
 FS_BY = {"cfg2": 100e6, "cfg3": 200e6, "cfg4": 50e6, "cfg5": 100e6}
@@ -230,10 +234,12 @@ def cpu_lib(kind):
     odir = os.path.join(ROOT, "oracle")
     path = {"fast": "libsdoracle_fast.so", "native": "libsdoracle_native.so", "parity": "libsdoracle.so"}[kind]
     path = os.path.join(odir, "_build", path)
-    if kind == "native" and not os.path.exists(path):
-        subprocess.run(["make", "-C", odir, "native"], capture_output=True)
-    if kind == "fast" and not os.path.exists(path):
-        subprocess.run(["make", "-C", odir], capture_output=True)
+    tmp = None
+    if kind in ("native", "fast") and not os.path.exists(path):
+        # built in a temporary directory, not in the tree (which may be read-only); removed once loaded
+        tmp = tempfile.mkdtemp(prefix="sdb_oracle_")
+        path = os.path.join(tmp, os.path.basename(path))
+        subprocess.run(["make", "-C", odir, path, "%s=%s" % (kind.upper(), path)], capture_output=True)
     L = None
     if os.path.exists(path):
         try:
@@ -244,6 +250,8 @@ def cpu_lib(kind):
             L.sdo_set_fast_transforms(0 if kind == "parity" else 1)
         except OSError:
             L = None
+    if tmp:
+        shutil.rmtree(tmp, ignore_errors=True)
     _CPU_LIBS[kind] = L
     return L
 
@@ -518,6 +526,9 @@ def run_cuda_cfg5(args):
         step_dev()
     with Clocks(local) as clk:
         ms = run(step_dev, args.steps, small)
+    if args.dump_outputs and rank == 0:
+        psd, accum, count = p.read()                # the stitched SpectrumView of the last sweep
+        write_dump(args.dump_outputs, {"view_psd": psd, "view_psd_accum": accum, "view_psd_count": count})
     samples = CFG5_HOPS * N_FFT
     value = samples * args.steps / (ms * 1e-3) / 1e6
     tm = p.timing()
@@ -614,6 +625,47 @@ def cfg5_cpu(n_hops):
 
 
 # --------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path handed back in its last step, so that two builds can be compared output for
+# output (inputs are seeded: the same arguments give the same inputs)
+# --------------------------------------------------------------------------------------------------
+DUMP_LIMIT = 64 << 20         # bytes written in all
+DUMP_STREAMS_BUDGET = 48 << 20
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte bound" % (total, DUMP_LIMIT))
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def dump_engine_outputs(out_dir, e, hs):
+    """PSD frames [streams, frames, N] and every inspector's soft / hard symbols of the last feed, for a fixed seeded
+    sample of the streams (all of them when they fit the budget); the sampled stream indices go with them."""
+    psd = e.read_psd()
+    S = psd.shape[0]
+    sym0 = sum(len(e.read_symbols(0, h)[1]) for h in hs)
+    per_stream = psd[0].nbytes + sym0 * 12                       # soft as 2 x float32, hard as float32
+    k = min(S, max(1, DUMP_STREAMS_BUDGET // max(1, per_stream)))
+    idx = np.arange(S) if k == S else np.sort(np.random.default_rng(0).choice(S, k, replace=False))
+    soft, hard, counts = [], [], np.zeros((k, len(hs)), np.float64)
+    for i, s in enumerate(idx):
+        for j, h in enumerate(hs):
+            sf, hd = e.read_symbols(int(s), h)
+            soft.append(sf)
+            hard.append(hd)
+            counts[i, j] = len(hd)
+    soft = np.concatenate(soft) if soft else np.zeros(0, np.complex64)
+    hard = np.concatenate(hard) if hard else np.zeros(0, np.uint8)
+    write_dump(out_dir, {"psd": psd[idx], "soft_symbols": soft.view(np.float32).reshape(-1, 2),
+                         "hard_symbols": hard.astype(np.float32), "symbol_counts": counts,
+                         "streams": idx.astype(np.float64)})
+
+
+# --------------------------------------------------------------------------------------------------
 # CUDA arm
 # --------------------------------------------------------------------------------------------------
 def build_engine(sdb, name, streams, n, device):
@@ -698,6 +750,8 @@ def run_cuda(args):
     with Clocks(local) as clk:
         ms = timed(step_dev, args.steps)
     launches = e.launches - l0
+    if args.dump_outputs and rank == 0:
+        dump_engine_outputs(args.dump_outputs, e, hs)
     value = samples_step * world * args.steps / (ms * 1e-3) / 1e6
 
     # ---- per-kernel device times: a separate pass in the engine's timing mode, which queues every kernel on ONE
@@ -908,6 +962,8 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-single", action="store_true")
     ap.add_argument("--no-formats", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="CUDA arm: write the outputs of the last timed step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
     global FS, N_FFT
     FS = FS_BY[args.workload]

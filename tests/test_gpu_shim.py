@@ -111,17 +111,12 @@ def test_analyzer_session_through_the_suscan_names(tu, oracle):
 
 
 def test_lpf_task_of_the_reference_over_the_specttuner_shim(oracle, sdb):
-    """Tasks/LPFTask.cpp COMPILED FROM THE REFERENCE (oracle/_ref/libsdref.so; su_specttuner_new / open_channel with
-    guard = 2 pi / bw / feed_bulk / the zero flush of :104-107) over <sigutils/specttuner.h>, whose tuner is an engine on
-    the GPU: same output as the engine's own LPF task and as the reference-shaped TU."""
+    """Tasks/LPFTask.cpp COMPILED FROM THE REFERENCE (su_specttuner_new / open_channel with guard = 2 pi / bw /
+    feed_bulk / the zero flush of :104-107) over <sigutils/specttuner.h>, whose tuner is an engine on the GPU: its
+    output, recorded in tests/golden/ref_compiled.json (tests/golden/record_ref.py --gpu), is the engine's own LPF
+    task's, bit for bit."""
     import os
-    so = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libsdref.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/libsdref.so not built (needs /root/reference at build time)")
-    R = C.CDLL(so)
-    R.ref_task_lpf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_float]
-    n = 5 * 4096 + 300
-    x = _sig(n, seed=9)
-    y = np.zeros(n, np.complex64)
-    assert R.ref_task_lpf(x.ctypes.data, y.ctypes.data, n, C.c_float(0.2)) == 0
-    assert np.array_equal(y.view(np.uint32), sdb.lpf(x, 0.2).view(np.uint32))
+    import sys
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+    import record_ref as R
+    assert R.same(R.load()["lpf"], sdb.lpf(R.lpf_input(), 0.2))
