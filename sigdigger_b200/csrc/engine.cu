@@ -718,6 +718,8 @@ extern "C" int sdb_engine_commit(sdb_engine_t *e)
     for (auto &kv : by_size) {
       sdb_engine::Group g; g.size = kv.first; g.len = (int) kv.second.size(); g.any_precise = 0;
       for (int id : kv.second) if (e->h_chans[id].precise) g.any_precise = 1;
+      if (!sdb_chan_ifft_fits(g.size, g.any_precise))     // fail here rather than at every feed
+        return fail("channel inverse transform of this size does not fit in shared memory");
       g.d_ids = e->dalloc<int>(kv.second.size());
       if (!g.d_ids) return fail("out of device memory");
       CK(cudaMemcpy(g.d_ids, kv.second.data(), kv.second.size() * sizeof(int), cudaMemcpyHostToDevice));

@@ -504,6 +504,10 @@ cudaError_t sdb_launch_spectsrc(const SdbLaunchCtx &c, const SdbSpectCfg *cfg_de
 // barrier of the shared-memory transform paid once per P hops, P gathers in flight -- and cross-fades them from the
 // buffers of their left neighbours; the last hop's second half is carried in shared memory (and between feeds in
 // `tails`).  Round 1 ran one hop at a time with size/4 threads: 22 us per 2048-point hop against < 1 us of work.
+// BPT > 1 (8192 and 16384 points, one hop per pass) carries that half window in `tails` itself: a 16384-point
+// channel's transform buffer, two shared half windows and the LO phases would need 288 KB, over the 227 KB a CTA
+// can have.  Each thread reads and rewrites only its own tail entries, so the global carry needs no barrier.
+// The LO phase array is only present when the group has a precise channel (launcher's `any_precise`).
 // ---------------------------------------------------------------------------------------------
 template <int BPT>
 __global__ void __launch_bounds__(1024) k_chan_ifft(const SdbChannelDev *__restrict__ chans,
@@ -513,21 +517,23 @@ __global__ void __launch_bounds__(1024) k_chan_ifft(const SdbChannelDev *__restr
                                                      size_t tail_stream_stride, float *__restrict__ lo_phase,
                                                      float2 *__restrict__ chan_out, size_t chan_stream_stride)
 {
+  constexpr bool kSmemTail = BPT == 1;
   extern __shared__ float2 sm[];
   const int ci = group[blockIdx.x];
   const SdbChannelDev ch = chans[ci];
   const int s = blockIdx.y;
   const int size = ch.size, hs = ch.halfsz, hw = ch.halfw;
   float2 *bufs = sm;                                   // [P][size]
-  float2 *prevb[2] = { sm + (size_t) P * size, sm + (size_t) P * size + hs };
-  float *phase = reinterpret_cast<float *>(sm + (size_t) P * size + 2 * hs);   // [P][hs]
+  float2 *prevb[2] = { sm + (size_t) P * size, sm + (size_t) P * size + hs };   // BPT = 1 only
+  float *phase = reinterpret_cast<float *>(sm + (size_t) P * size + (kSmemTail ? 2 * hs : 0));   // [P][hs]
   const int tid = threadIdx.x;
   const int per = BPT == 1 ? (size >= 4 ? size >> 2 : 1) : (int) blockDim.x;   // threads per hop
   const int g = tid / per, l = tid - g * per;
   float2 *__restrict__ tail = tails + (size_t) s * tail_stream_stride + ch.tail_off;
   float2 *__restrict__ out = chan_out + (size_t) s * chan_stream_stride + ch.out_off;
 
-  for (int i = tid; i < hs; i += blockDim.x) prevb[0][i] = tail[i];
+  if (kSmemTail)
+    for (int i = tid; i < hs; i += blockDim.x) prevb[0][i] = tail[i];
   float lo_phi = ch.precise ? lo_phase[(size_t) s * n_channels + ci] : 0.0f;
   int pb = 0;
   __syncthreads();
@@ -563,7 +569,7 @@ __global__ void __launch_bounds__(1024) k_chan_ifft(const SdbChannelDev *__restr
     __syncthreads();
     block_fft_inplace<+1, BPT>(buf, size, ch.log2size, active ? l : size, per, ch.tw);
     if (active) {
-      const float2 *pvb = g > 0 ? buf - size + hs : prevb[pb];
+      const float2 *pvb = g > 0 ? buf - size + hs : (kSmemTail ? prevb[pb] : tail);
       for (int i = l; i < hs; i += per) {
         const float al = __ldg(ch.xfade + i), be = __ldg(ch.xfade + i + hs);
         const float2 cu = buf[i], pv = pvb[i];
@@ -574,13 +580,17 @@ __global__ void __launch_bounds__(1024) k_chan_ifft(const SdbChannelDev *__restr
           o = cmulc(o, make_float2(cs_, sn));
         }
         out[(size_t) (j0 + g) * hs + i] = o;
-        if (g == Pg - 1) prevb[pb ^ 1][i] = buf[i + hs];
+        if (g == Pg - 1) {
+          if (kSmemTail) prevb[pb ^ 1][i] = buf[i + hs];
+          else tail[i] = buf[i + hs];
+        }
       }
     }
     pb ^= 1;
     __syncthreads();
   }
-  for (int i = tid; i < hs; i += blockDim.x) tail[i] = prevb[pb][i];
+  if (kSmemTail)
+    for (int i = tid; i < hs; i += blockDim.x) tail[i] = prevb[pb][i];
   if (ch.precise && tid == 0) lo_phase[(size_t) s * n_channels + ci] = lo_phi;
 }
 
@@ -785,41 +795,21 @@ k_chan_ifft16(const SdbChannelDev *__restrict__ chans, const int *__restrict__ g
   if (any_precise && ch.precise && tid == IFFT16_THREADS - 1) lo_phase[(size_t) s * n_channels + ci] = lo_phi;
 }
 
-// host side: channels grouped by size so that every CTA of a launch has the right block size
-cudaError_t sdb_launch_chan_ifft_group(const SdbLaunchCtx &c, const SdbChannelDev *chans_dev,
-                                       const int *group_dev, int group_len, int size, int n_channels,
-                                       int n_streams, const float2 *cspec, int n_bins, int wps,
-                                       float2 *tails, size_t tail_stream_stride, float *lo_phase,
-                                       float2 *chan_out, size_t chan_stream_stride, int any_precise)
+// host side: channels grouped by size so that every CTA of a launch has the right block size.  The launch shape of a
+// group depends only on its size, its hops per feed and whether it holds a precise channel.
+struct ChanIfftPlan { bool use16; int bpt, threads, P; size_t smem, smem_max; };
+
+static ChanIfftPlan chan_ifft_plan(int size, int wps, int any_precise)
 {
-  static std::atomic<unsigned long long> attr_done{ 0 };   // one bit per device: function attributes are per context
   static const int use16 = getenv("SDB_IFFT16") ? atoi(getenv("SDB_IFFT16")) : 1;
+  ChanIfftPlan q{};
+  const size_t phase_bytes = any_precise ? (size_t) (size / 2) * sizeof(float) : 0;   // per hop of a pass
   if (use16 && size >= 512 && size <= 4096) {
-    static std::atomic<unsigned long long> attr16_done{ 0 };
-    static const int occ = getenv("SDB_IFFT16_OCC") ? atoi(getenv("SDB_IFFT16_OCC")) : 3;
-    if (sdb_first_on_device(attr16_done)) {
-      cudaFuncSetAttribute(k_chan_ifft16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-      cudaFuncSetAttribute(k_chan_ifft16<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    }
-    const int per = size / 16, P = IFFT16_THREADS / per;
-    const size_t smem = (size_t) P * (size + size / 16) * sizeof(float2) + (size_t) size * sizeof(float2)
-                        + (any_precise ? (size_t) P * (size / 2) * sizeof(float) : 0);
-    dim3 grid(group_len, n_streams);
-    if (occ == 4)
-      k_chan_ifft16<4><<<grid, IFFT16_THREADS, smem, c.stream>>>(chans_dev, group_dev, n_channels, cspec, n_bins, wps,
-                                                                 any_precise, tails, tail_stream_stride, lo_phase,
-                                                                 chan_out, chan_stream_stride);
-    else
-      k_chan_ifft16<3><<<grid, IFFT16_THREADS, smem, c.stream>>>(chans_dev, group_dev, n_channels, cspec, n_bins, wps,
-                                                                 any_precise, tails, tail_stream_stride, lo_phase,
-                                                                 chan_out, chan_stream_stride);
-    if (c.launch_counter) ++*c.launch_counter;
-    return cudaGetLastError();
-  }
-  if (sdb_first_on_device(attr_done)) {
-    cudaFuncSetAttribute(k_chan_ifft<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(k_chan_ifft<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(k_chan_ifft<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    const int per = size / 16;
+    q.use16 = true; q.bpt = 1; q.threads = IFFT16_THREADS; q.P = IFFT16_THREADS / per;
+    q.smem = (size_t) q.P * (size + size / 16) * sizeof(float2) + (size_t) size * sizeof(float2) + q.P * phase_bytes;
+    q.smem_max = 100 * 1024;
+    return q;
   }
   int bpt = 1, threads = size / 4;
   while (threads > 1024) { threads >>= 1; bpt <<= 1; }
@@ -840,9 +830,55 @@ cudaError_t sdb_launch_chan_ifft_group(const SdbLaunchCtx &c, const SdbChannelDe
     threads = size / 4;
   }
   if (threads < 32) threads = 32;
-  const size_t smem = (size_t) P * size * sizeof(float2) + (size_t) size * sizeof(float2)
-                      + (size_t) P * (size / 2) * sizeof(float);
-  if (smem > 200 * 1024) return cudaErrorInvalidValue;
+  q.use16 = false; q.bpt = bpt; q.threads = threads; q.P = P;
+  // P transform buffers, the two carried half windows when they live in shared memory (BPT = 1), the LO phases
+  q.smem = (size_t) P * size * sizeof(float2) + (bpt == 1 ? (size_t) size * sizeof(float2) : 0) + P * phase_bytes;
+  q.smem_max = 200 * 1024;
+  return q;
+}
+
+// whether a group of `size`-point channels can be launched, for any number of hops per feed
+bool sdb_chan_ifft_fits(int size, int any_precise)
+{
+  const ChanIfftPlan q = chan_ifft_plan(size, 1 << 30, any_precise);
+  return q.smem <= q.smem_max && (q.use16 || q.bpt <= 4);
+}
+
+cudaError_t sdb_launch_chan_ifft_group(const SdbLaunchCtx &c, const SdbChannelDev *chans_dev,
+                                       const int *group_dev, int group_len, int size, int n_channels,
+                                       int n_streams, const float2 *cspec, int n_bins, int wps,
+                                       float2 *tails, size_t tail_stream_stride, float *lo_phase,
+                                       float2 *chan_out, size_t chan_stream_stride, int any_precise)
+{
+  static std::atomic<unsigned long long> attr_done{ 0 };   // one bit per device: function attributes are per context
+  const ChanIfftPlan q = chan_ifft_plan(size, wps, any_precise);
+  if (q.smem > q.smem_max) return cudaErrorInvalidValue;
+  const size_t smem = q.smem;
+  if (q.use16) {
+    static std::atomic<unsigned long long> attr16_done{ 0 };
+    static const int occ = getenv("SDB_IFFT16_OCC") ? atoi(getenv("SDB_IFFT16_OCC")) : 3;
+    if (sdb_first_on_device(attr16_done)) {
+      cudaFuncSetAttribute(k_chan_ifft16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+      cudaFuncSetAttribute(k_chan_ifft16<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+    }
+    dim3 grid(group_len, n_streams);
+    if (occ == 4)
+      k_chan_ifft16<4><<<grid, IFFT16_THREADS, smem, c.stream>>>(chans_dev, group_dev, n_channels, cspec, n_bins, wps,
+                                                                 any_precise, tails, tail_stream_stride, lo_phase,
+                                                                 chan_out, chan_stream_stride);
+    else
+      k_chan_ifft16<3><<<grid, IFFT16_THREADS, smem, c.stream>>>(chans_dev, group_dev, n_channels, cspec, n_bins, wps,
+                                                                 any_precise, tails, tail_stream_stride, lo_phase,
+                                                                 chan_out, chan_stream_stride);
+    if (c.launch_counter) ++*c.launch_counter;
+    return cudaGetLastError();
+  }
+  if (sdb_first_on_device(attr_done)) {
+    cudaFuncSetAttribute(k_chan_ifft<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(k_chan_ifft<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(k_chan_ifft<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  }
+  const int bpt = q.bpt, threads = q.threads, P = q.P;
   dim3 grid(group_len, n_streams);
   if (bpt == 1)
     k_chan_ifft<1><<<grid, threads, smem, c.stream>>>(chans_dev, group_dev, n_channels, cspec, n_bins, wps, P,

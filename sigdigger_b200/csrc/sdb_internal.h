@@ -258,6 +258,7 @@ cudaError_t sdb_launch_chan_ifft_group(const SdbLaunchCtx &c, const SdbChannelDe
                                        int n_streams, const float2 *cspec, int n_bins, int wps,
                                        float2 *tails, size_t tail_stream_stride, float *lo_phase,
                                        float2 *chan_out, size_t chan_stream_stride, int any_precise = 1);
+bool sdb_chan_ifft_fits(int size, int any_precise);
 cudaError_t sdb_launch_sym_pack(cudaStream_t stream, const uint32_t *counts, unsigned long long *offsets, size_t chains,
                                 const float2 *soft, const unsigned char *hard, size_t cap, void *out_soft,
                                 void *out_hard, unsigned long long cap_total, uint64_t *launch_counter);
